@@ -1,6 +1,7 @@
 """bench.py — benchmark of the SO-Net forward hot path on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config cfg2]
+                    [--dump-outputs DIR]
 
 Default (--config cfg2, BASELINE.json configs[1], the headline): a "step" is one eval-mode
 classifier forward (ModelNet40 shape: batch 64 per GPU, N=5000 points, 8x8 SOM, k=3, som_k=9,
@@ -28,6 +29,10 @@ line.
             host cores on a bounded sample (8 clouds of this run's inputs). Its outputs are also
             the parity check of the timed GPU steps ("parity")
   --impl reference   only that CPU arm, same JSON shape with "impl": "reference"
+  --dump-outputs DIR   after the timed steps, rank 0 writes what the last timed step handed its
+            caller (the task's Model outputs, step_outputs()) as DIR/<name>.npy, float32. Inputs
+            and weights are seeded, so two builds run with the same arguments can be compared
+            array by array.
 """
 import argparse
 import json
@@ -181,6 +186,36 @@ def result_rows(task, model):
                         model.chamfer_criteria.backward_loss_array), dim=1)   # [B, 2]
 
 
+DUMP_BUDGET = 64 << 20       # bytes that --dump-outputs writes, all arrays together
+
+
+def step_outputs(task, model):
+    """What a caller reads from the Model after test_model() (models/<task>.py), as float32
+    host copies."""
+    names = {"classifier": ("score", "feature", "loss"),
+             "segmenter": ("score_segmenter", "feature", "loss"),
+             "autoencoder": ("predicted_pc", "feature", "loss_chamfer", "loss_chamfer_conv4",
+                             "loss")}[task]
+    out = {n: getattr(model, n) for n in names if torch.is_tensor(getattr(model, n, None))}
+    if task == "autoencoder":
+        out["chamfer_loss_arrays"] = result_rows(task, model)
+    return {n: t.detach().float().cpu() for n, t in out.items()}
+
+
+def dump_outputs(path, arrays):
+    """Write each array as <path>/<name>.npy. An array larger than its share of DUMP_BUDGET is
+    written as a sample of its flattened elements at positions drawn from a fixed seed, so that
+    two runs sample the same positions."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    share = DUMP_BUDGET // (4 * len(arrays))                  # float32 elements per array
+    for name, t in arrays.items():
+        if t.numel() > share:
+            g = torch.Generator().manual_seed(0)
+            t = t.reshape(-1)[torch.randperm(t.numel(), generator=g)[:share].sort().values]
+        np.save(os.path.join(path, name + ".npy"), t.numpy())
+
+
 # ---- CPU arm: the reference's own PyTorch-CPU path ---------------------------------------------------
 def _cpu_step_fn(cfg, sample_B, inp, st_e, st_h):
     """Returns (step() -> result rows [sample_B, ...], set_threads(n), kind, description).
@@ -285,7 +320,7 @@ def cpu_arm(cfg, steps, warmup, sample_B=8, inp=None):
 def run_reference_arm(args, rank, cfg):
     if rank != 0:
         return
-    steps = max(1, min(args.steps, 5))
+    steps = args.steps
     warm = max(1, min(args.warmup, 2))
     cb, _ = cpu_arm(cfg, steps, warm)
     line = {"impl": "reference", "metric": cfg["metric"], "value": cb["value"], "unit": UNIT,
@@ -476,7 +511,13 @@ def main():
                          "sonet_allgather (the same NCCL, resolved by libsonet_b200)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="eager op calls instead of CUDA-graph replay")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; --impl reference has none")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
     cfg = CONFIGS[args.config]
     task, B, NPTS = cfg["task"], cfg["B"], cfg["N"]
@@ -574,6 +615,11 @@ def main():
     wall = time.perf_counter() - wall0
     timed_rows = result_rows(task, model).detach().clone()  # result of the last timed step
     timed_gather = out.detach().clone()
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        dumped = step_outputs(task, model)
+        if world > 1:
+            dumped["gathered_rows"] = timed_gather.float().cpu()
     launches = ops.KERNEL_LAUNCHES - l0
     step_ms = [a.elapsed_time(b) for a, b in evs]
     total_ms = torch.tensor([sum(step_ms)], dtype=torch.float64, device=dev)
@@ -724,6 +770,8 @@ def main():
                 "parity_checked": bool(parity and parity["ok"]),
                 "gather_check": gather_check,
                 "checksum": float(timed_gather.double().sum().item())}
+        if dumped:
+            dump_outputs(args.dump_outputs, dumped)
         print(json.dumps(line))
     if world > 1:
         dist.barrier()

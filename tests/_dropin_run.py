@@ -3,9 +3,9 @@ sys.modules, so it must not run inside the pytest process).
 
     python tests/_dropin_run.py <reference_root> <device>
 
-Imports the REFERENCE's own models/{classifier,segmenter,autoencoder}.py — from /root/reference
-(build container) or from the bytecode build product oracle/_ref/pyref (GPU box) — on top of
-sonet_b200's networks/layers/losses/som/index_max, and on a CUDA device runs their unmodified
+Imports the REFERENCE's own models/{classifier,segmenter,autoencoder}.py — from the bytecode
+build product oracle/_ref/pyref — on top of sonet_b200's networks/layers/losses/som/index_max,
+and on a CUDA device runs their unmodified
 Model.set_input()/test_model() against the golden vectors the reference itself produced."""
 import os
 import sys
